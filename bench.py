@@ -13,7 +13,13 @@ same through the C ABI with pinned HOST buffers (H2D of the operands and D2H of 
 the timed region); roofline = dominant kernel vs the measured HBM peak; cpu_baseline = the C++
 oracle (restated NTL-path HElib) on the host cores.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes, after the timed steps, the two result parts c0 and c1 the timed path left in HBM (rows of the
+19 ctxt primes) as DIR/c0.npy and DIR/c1.npy: float64 arrays [batch][19][columns][2] holding each 60-bit residue as
+(high 32 bits, low 32 bits), both exact in float64, over a fixed seeded sample of coefficient columns that keeps the
+two files under 64 MB together.  The inputs depend only on the arguments, so two builds run with the same arguments
+can be compared file for file.
 """
 import argparse
 import json
@@ -29,6 +35,8 @@ sys.path.insert(0, ROOT)
 WORKLOAD = {"name": "ckks_m2^17_bits1190_c2", "m": 1 << 17, "p": -1, "r": 1, "bits": 1190, "c": 2}
 SEED = 20260922 + 2  # SURVEY 8d: Philox, seed = 20260922 + config index
 ROW_BYTES = (1 << 16) * 8
+DUMP_BYTES = 63 * 10**6    # --dump-outputs: data of all files together (under 64 MB with the .npy headers)
+DUMP_COLUMNS = 2048        # --dump-outputs: sampled coefficient columns per row (fewer when the batch is large)
 
 
 def alg_bytes_per_mult(l_in, l, K, d):
@@ -117,6 +125,24 @@ def mult_config(B):
             "l2": f"inputs larger than L2 ({B * 4 * l_in * ROW_BYTES / 2**20:.0f} MiB of operands per step)",
             "operands": "updated in place: from step 2 on a step's inputs are the previous step's outputs (the path is data-oblivious)",
             "alg_bytes_per_mult": alg_bytes_per_mult(l_in, l, K, d)}
+
+
+def dump_columns(N, B, l):
+    """The coefficient columns --dump-outputs keeps: a sorted sample, fixed by SEED, sized so that two parts of B x l rows
+    at 16 bytes per residue fit DUMP_BYTES."""
+    import numpy as np
+    n = max(1, min(N, DUMP_COLUMNS, DUMP_BYTES // (2 * B * l * 16)))
+    return np.sort(np.random.Generator(np.random.Philox(SEED)).choice(N, size=n, replace=False))
+
+
+def dump_outputs(path, parts, S, N):
+    """Write each named list of result polys as path/<name>.npy (layout in the module docstring)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    cols = dump_columns(N, len(next(iter(parts.values()))), len(S))
+    for name, polys in parts.items():
+        res = np.stack([p.download(S)[S][:, cols] for p in polys])
+        np.save(os.path.join(path, name + ".npy"), np.stack([res >> np.uint64(32), res & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64))
 
 
 def cpu_layout(cores):
@@ -520,7 +546,10 @@ def main():
     ap.add_argument("--ks-group", type=int, default=64, help="config 3: ciphertexts per hb_relinearize / hb_scale_down call")
     ap.add_argument("--ks-steps", type=int, default=3, help="config 3: timed passes over the resident ciphertexts (at most --steps)")
     ap.add_argument("--sharded-batch", type=int, default=32, help="config 4: ciphertexts per step of the prime-sharded key switch")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the results of the last one as DIR/c0.npy, DIR/c1.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if args.warmup < 3:
@@ -610,6 +639,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = world * B * args.steps / (ms / 1000.0)
+    if args.dump_outputs and rank == 0:     # before the e2e loop, which reuses these polys
+        dump_outputs(args.dump_outputs, {"c0": A0, "c1": A1}, S, N)
 
     # ---- e2e: host buffers -> H2D -> hot path -> D2H, every step.  Two engine contexts (two CUDA
     #      streams), each with half of the batch, so the PCIe copies of one half overlap the kernels of

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -48,6 +50,50 @@ def test_both_arms_describe_the_same_workload():
     for cores in (1, 8, 16, 128, 192):
         w, per = bench.cpu_layout(cores)
         assert w >= 1 and per >= 1 and w * per <= max(cores, 1)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(cuda_lib, tmp_path):
+    """--dump-outputs: the files hold, bit for bit, what warm-up + --steps in-place multiplies of the seeded inputs leave in
+    c0 and c1 (replayed here through the engine), on the documented column sample and within the size budget."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from helib_b200 import Chain, Engine
+    B, warmup, steps = 2, 3, 2
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", str(warmup), "--batch", str(B),
+                        "--no-cpu", "--no-e2e", "--no-ks", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+    assert sorted(os.listdir(tmp_path)) == ["c0.npy", "c1.npy"]
+    assert sum(os.path.getsize(tmp_path / f) for f in os.listdir(tmp_path)) <= 64 * 10**6
+
+    w = bench.WORKLOAD
+    ch = Chain(w["m"], w["p"], w["r"], w["bits"], w["c"], lib=cuda_lib)
+    E = Engine(w["m"], ch.primes, None, ch.digits, ch.special, lib=cuda_lib)
+    S_in, S, full = ch.ctxt, ch.ctxt[:-1], ch.ctxt + ch.special
+    rng = np.random.Generator(np.random.Philox(bench.SEED))
+
+    def rand_dense(idx):
+        out = np.zeros((E.np, E.N), dtype=np.uint64)
+        for i in idx:
+            out[i] = rng.integers(0, ch.primes[i], size=E.N, dtype=np.uint64)
+        return out
+
+    EA = [E.poly(rand_dense(full), full) for _ in ch.digits]
+    EB = [E.poly(rand_dense(full), full) for _ in ch.digits]
+    ops = [[E.poly(rand_dense(S_in), S_in) for _ in range(4)] for _ in range(B)]
+    A0, A1, B0, B1 = ([o[k] for o in ops] for k in range(4))
+    for _ in range(warmup + steps):
+        E.mul_relin_moddown(A0, A1, B0, B1, S_in, S, 1, EA, EB)
+    cols = bench.dump_columns(E.N, B, len(S))
+    for name, polys in (("c0", A0), ("c1", A1)):
+        got = np.load(tmp_path / (name + ".npy"))
+        assert got.dtype == np.float64 and got.shape == (B, len(S), len(cols), 2)
+        want = np.stack([p.download(S)[S][:, cols] for p in polys])
+        assert (((got[..., 0].astype(np.uint64) << np.uint64(32)) | got[..., 1].astype(np.uint64)) == want).all(), name
+    del A0, A1, B0, B1, ops, EA, EB
+    E.close()
 
 
 def test_product_arm_refuses_to_run_without_a_gpu():
